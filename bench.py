@@ -84,7 +84,12 @@ def parse():
                         "checkpoint whisper would fall back to all heads of the upper half of the decoder)")
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--ncu", action="store_true", help="profiling run: warm up, then ONE step inside cudaProfilerStart/Stop")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32 / float64), "
+                        "so that two builds can be compared output for output on the same seeded inputs")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
     if a.tokens is None:
         a.tokens = 224 if a.workload == "transcribe" else 100
     if a.workload == "refine" and a.windows == 120:
@@ -406,6 +411,46 @@ def ncu_traffic(kernel: str, algorithmic_bytes_per_launch: float):
     return None, None
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, workload, step_out):
+    """What one device step returned, as flat arrays in window order (every output of these workloads is far below
+    DUMP_LIMIT_BYTES, so nothing is sampled):
+      transcribe: per word its window, start, end, probability and tokens (padded with -1 to the longest word), and the
+                  token argmax of every decode step [steps, windows];
+      align:      per window the DTW jump indices and the text-token probabilities, concatenated, with per-window lengths;
+      refine:     per group the probabilities and ranks [2, N] of its script, concatenated along N, with per-group lengths."""
+    arrays = {}
+    if workload == "transcribe":
+        segs, info = step_out
+        words = [(b, w) for b, ws in enumerate(segs) for s_ in ws for w in s_["words"]]
+        width = max([len(w["tokens"]) for _, w in words] + [1])
+        arrays["word_window"] = np.array([b for b, _ in words], dtype=np.float64)
+        for k in ("start", "end", "probability"):
+            arrays[f"word_{k}"] = np.array([w[k] for _, w in words], dtype=np.float64)
+        arrays["word_tokens"] = np.array([list(w["tokens"]) + [-1] * (width - len(w["tokens"])) for _, w in words],
+                                         dtype=np.float64).reshape(len(words), width)
+        sa = info["step_argmax"]
+        arrays["step_argmax"] = (sa.cpu().numpy() if torch.is_tensor(sa) else np.asarray(sa)).astype(np.float64)
+    elif workload == "align":
+        arrays["jumps"] = np.concatenate([np.asarray(j) for j, _ in step_out]).astype(np.float64)
+        arrays["jumps_len"] = np.array([len(j) for j, _ in step_out], dtype=np.float64)
+        arrays["token_probs"] = np.concatenate([np.asarray(p, dtype=np.float64) for _, p in step_out])
+        arrays["token_probs_len"] = np.array([len(p) for _, p in step_out], dtype=np.float64)
+    else:
+        arrays["probs"] = torch.cat([p.float().cpu() for p, _ in step_out], dim=1).numpy()
+        arrays["ranks"] = torch.cat([r.cpu() for _, r in step_out], dim=1).numpy().astype(np.float64)
+        arrays["group_len"] = np.array([p.shape[1] for p, _ in step_out], dtype=np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py --dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print(f"[bench] dumped {len(arrays)} arrays ({total} bytes) to {out_dir}", file=sys.stderr)
+
+
 # ------------------------------------------------------------------------------------------------- B200 arm
 def run_b200(args, dims_tuple):
     import torch.distributed as dist
@@ -523,7 +568,7 @@ def run_b200(args, dims_tuple):
     marks = [torch.cuda.Event(enable_timing=True) for _ in range(args.steps)]
     e0.record()
     for i in range(args.steps):
-        device_step(i % pools)
+        last = device_step(i % pools)
         marks[i].record()
     e1.record()
     barrier()
@@ -531,6 +576,9 @@ def run_b200(args, dims_tuple):
     ms = e0.elapsed_time(e1)
     step_ms = [round(a.elapsed_time(b), 1) for a, b in zip([e0] + marks[:-1], marks)]    # per-step spread (rank 0)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, args.workload, last)
+    del last
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -64,10 +64,10 @@ class Segment:                        # stable_whisper/result.py Segment
             self._sync()
 
     def _sync(self):
-        if self.words:                # a segment with words takes its text and span from them (result.py Segment.text/start/end)
-            self.text = "".join(w.word for w in self.words)
+        if self.words:                # a segment with words takes its text, span and tokens from them (result.py Segment.text/
+            self.text = "".join(w.word for w in self.words)     # start/end/tokens: the timestamp tokens are not listed)
             self.start, self.end = self.words[0].start, self.words[-1].end
-            if self.tokens is None and all(w.tokens is not None for w in self.words):
+            if self.words[0].tokens:
                 self.tokens = [t for w in self.words for t in w.tokens]
 
     @property

@@ -3,8 +3,12 @@
 ``stable_ts_b200``'s plugin closures and bound model methods, with an oracle-backed stand-in for the GPU model's method
 surface (tests/standin.py).  Every result must be IDENTICAL to what the reference's own entry points
 (``stable_whisper.alignment.align / align_words / refine``) produce with their vanilla closures over the same oracle
-model.  Skipped where the reference tree is absent (GPU box: tests/test_gpu_boundary.py covers the real kernels)."""
+model.  The tests that drive ``Aligner`` / ``Refiner`` run the reference package itself, installed into oracle/_ref/ by
+``build()`` (oracle/reference_install.py), and skip where it could not be installed;
+``locate`` and the result schema are compared with what the reference returned (tests/golden/reference_results.json, written
+by oracle/make_golden_reference.py).  tests/test_gpu_boundary.py covers the real kernels."""
 import copy
+import json
 import os
 import sys
 
@@ -12,17 +16,12 @@ import numpy as np
 import pytest
 import torch
 
-REFERENCE = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference tree only exists in the build container")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_results.json")
 
 
 @pytest.fixture(scope="module")
 def env():
     import oracle.whisper_ref as W
-    W.install_as_whisper()
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-    import stable_whisper  # noqa: F401
     from oracle import stable_path as SP
     from standin import OracleBackedModel
     model = W.build_model("tiny", seed=5)
@@ -30,7 +29,28 @@ def env():
     audio = torch.cat([SP.synth_gapped_audio(400000, seed=11), SP.synth_audio(300000, seed=12)])
     words = SP.words_from_script(SP.synth_token_script(70, tk.eot, seed=13))
     text = "".join(tk.decode(w) for w in words)
-    return dict(W=W, SP=SP, model=model, tk=tk, audio=audio, text=text, stand=OracleBackedModel(model))
+    with open(GOLD) as f:
+        gold = json.load(f)["boundary"]
+    return dict(W=W, SP=SP, model=model, tk=tk, audio=audio, text=text, stand=OracleBackedModel(model), gold=gold)
+
+
+@pytest.fixture(scope="module")
+def ref_env(env):
+    """The reference package importable (from oracle/_ref/) for the rest of this module, and no longer afterwards: the
+    other modules test this package's own result classes."""
+    from oracle import reference_install
+    root = reference_install.path()
+    env["W"].install_as_whisper()             # the reference imports `whisper`; the oracle restates it
+    if root is not None:
+        sys.path.insert(0, root)
+    try:
+        pytest.importorskip("stable_whisper", reason="the reference package (stable-ts) is not installed in oracle/_ref/")
+        yield env
+    finally:
+        if root is not None:
+            sys.path.remove(root)
+            for name in [m for m in sys.modules if m == "stable_whisper" or m.startswith("stable_whisper.")]:
+                del sys.modules[name]
 
 
 def _same_result(a, b, prob_tol=1e-5):
@@ -46,7 +66,8 @@ def _same_result(a, b, prob_tol=1e-5):
             assert abs(wa["probability"] - wb["probability"]) <= prob_tol * max(abs(wb["probability"]), 1e-30)
 
 
-def test_align_through_unmodified_aligner_is_identical(env):
+def test_align_through_unmodified_aligner_is_identical(ref_env):
+    env = ref_env
     import stable_whisper.alignment as ref_align
     from stable_ts_b200 import api
     theirs = ref_align.align(env["model"], env["audio"], env["text"], language="en", verbose=None, ignore_compatibility=True)
@@ -57,7 +78,8 @@ def test_align_through_unmodified_aligner_is_identical(env):
     assert env["stand"].calls["decode_forced"] >= 1
 
 
-def test_align_words_and_refine_through_unmodified_control_plane(env):
+def test_align_words_and_refine_through_unmodified_control_plane(ref_env):
+    env = ref_env
     import stable_whisper.alignment as ref_align
     from stable_ts_b200 import api
     base = ref_align.align(env["model"], env["audio"], env["text"], language="en", verbose=None, ignore_compatibility=True)
@@ -75,8 +97,9 @@ def test_align_words_and_refine_through_unmodified_control_plane(env):
     print(f"refine moved {moved} word boundaries; identical to the reference's vanilla closure")
 
 
-def test_refine_closure_3d_form_reaches_rank_test(env):
+def test_refine_closure_3d_form_reaches_rank_test(ref_env):
     """The closure returns the 3-D tensor, so ``Refiner.get_prob`` computes real token positions (refinement.py:305-325)."""
+    env = ref_env
     from stable_whisper.non_whisper.refinement import Refiner
     from stable_ts_b200.alignment import get_b200_refinement_func
     from stable_ts_b200.tokenizer import get_tokenizer
@@ -93,13 +116,13 @@ def test_refine_closure_3d_form_reaches_rank_test(env):
     assert pos == [int(rank[i % 2, i]) for i in range(len(script))] and any(p > 0 for p in pos)
 
 
-def test_own_result_schema_loads_in_the_reference(env):
-    """result.py stand-in <-> stable_whisper.WhisperResult: same dict schema both ways (result.py:618-636, :1398-1406)."""
+def test_own_result_schema_loads_in_the_reference(ref_env):
+    """result.py stand-in <-> stable_whisper.WhisperResult: same dict schema both ways (result.py:618-636, :1398-1406).  `d` is
+    what the reference's align() returned, as its to_dict(keep_orig=False) wrote it."""
     import stable_whisper
-    import stable_whisper.alignment as ref_align
     from stable_ts_b200.result import WhisperResult as Mine
-    theirs = ref_align.align(env["model"], env["audio"], env["text"], language="en", verbose=None, ignore_compatibility=True)
-    d = theirs.to_dict(keep_orig=False)         # with ori_dict kept, BOTH classes read `language` from it (result.py:938-939)
+    d = ref_env["gold"]["align_result"]         # with ori_dict kept, BOTH classes read `language` from it (result.py:938-939)
+    theirs = stable_whisper.WhisperResult(copy.deepcopy(d))
     mine = Mine(copy.deepcopy(d))
     again = stable_whisper.WhisperResult(mine.to_dict(keep_orig=False))
     _same_result(again, theirs, prob_tol=0)
@@ -116,26 +139,25 @@ def test_own_result_schema_loads_in_the_reference(env):
 def test_locate_matches_unmodified_reference(env, mode, thr):
     """stable_ts_b200.locate (host loop + kernel calls) over the stand-in == stable_whisper.alignment.locate over the oracle
     model (alignment.py:756-1116): target times (mode 2), confirmed segments with word timings (mode 0), window words (mode 1)."""
-    import stable_whisper.alignment as ref_align
     from stable_ts_b200 import api
     stand = api.modify_model(env["stand"])
     text = [700, 901, 333]
-    kw = dict(count=3, mode=mode, probability_threshold=thr, exact_token=True, max_token_per_seg=8, verbose=None)
-    theirs = ref_align.locate(env["model"], env["audio"], text, "en", **kw)
-    mine = stand.locate(env["audio"], text, "en", **{k: v for k, v in kw.items() if k != "verbose"})
+    kw = dict(count=3, mode=mode, probability_threshold=thr, exact_token=True, max_token_per_seg=8)
+    theirs = env["gold"]["locate"][f"{mode}|{thr}"]
+    mine = stand.locate(env["audio"], text, "en", **kw)
     assert len(mine) == len(theirs)
     if mode != 0 or thr == 0.0:
         assert len(mine) > 0
     for a, b in zip(mine, theirs):
         if mode == 2:
-            assert a == b
+            assert json.loads(json.dumps(a)) == b
         elif mode == 1:
             assert a["end"] == b["end"] and a["duration_window_text"] == b["duration_window_text"]
             assert [w["tokens"] for w in a["duration_window_word"]] == [w["tokens"] for w in b["duration_window_word"]]
             np.testing.assert_allclose([w["probability"] for w in a["duration_window_word"]],
                                        [w["probability"] for w in b["duration_window_word"]], rtol=1e-5)
         else:
-            da, db = a.to_dict(), b.to_dict()
+            da, db = a.to_dict(), b
             assert da["seek"] == db["seek"] and da["start"] == db["start"] and da["end"] == db["end"]
             assert [(w["word"], w["tokens"], w["start"], w["end"]) for w in da["words"]] == \
                    [(w["word"], w["tokens"], w["start"], w["end"]) for w in db["words"]]

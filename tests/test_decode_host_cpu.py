@@ -1,25 +1,26 @@
 """Host logic of the decode / transcribe drivers in the build container (SURVEY.md section 8 rows a9 + b): the batched engine's
 bookkeeping -- right-aligned ragged prompts, per-sequence n_ctx caps, best_of grouping and ranking, temperature-fallback
 subsets, prompt carry-over and reset, data-dependent seek -- over an oracle-backed stand-in for the model AND the step engine
-(tests/standin.py), compared with the UNMODIFIED ``transcribe_stable`` over the same oracle model.  The kernels behind the real
-engine are pinned by tests/test_gpu_sampling.py and tests/test_gpu_boundary.py on the GPU box."""
+(tests/standin.py), compared with what the UNMODIFIED ``transcribe_stable`` returned over the same oracle model
+(tests/golden/reference_results.json, written by oracle/make_golden_reference.py with the same inputs and uniforms).  The
+kernels behind the real engine are pinned by tests/test_gpu_sampling.py and tests/test_gpu_boundary.py on the GPU."""
+import json
 import os
-import sys
 
 import pytest
 import torch
 
-REFERENCE = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference tree only exists in the build container")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_results.json")
+
+
+def _golden(key):
+    with open(GOLD) as f:
+        return json.load(f)["transcribe"][key]
 
 
 @pytest.fixture(scope="module")
 def env():
     import oracle.whisper_ref as W
-    W.install_as_whisper()
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-    import stable_whisper  # noqa: F401
     from oracle import stable_path as SP
     from standin import OracleBackedModel, OracleStepEngine
     from stable_ts_b200 import api
@@ -41,8 +42,9 @@ def env():
             return None, None
         loud = [SIL.audio2loudness(a.numpy()) for a in audio]
         return np.stack([SIL.loudness_to_raw_mask(l, q_levels, k_size) for l in loud]), (np.stack(loud) if want_loudness else None)
-    sil.sound_masks = sound_masks
-    return dict(W=W, SP=SP, om=om, stand=stand, tk=tk)
+    with pytest.MonkeyPatch.context() as mp:          # undone after this module: the GPU tests call the real kernel
+        mp.setattr(sil, "sound_masks", sound_masks)
+        yield dict(W=W, SP=SP, om=om, stand=stand, tk=tk)
 
 
 def test_ragged_prompts_and_caps_match_oracle_window_by_window(env):
@@ -87,22 +89,6 @@ def test_ragged_prompts_and_caps_match_oracle_window_by_window(env):
     assert res[0].tokens == ref.tokens and abs(res[0].avg_logprob - ref.avg_logprob) < 1e-4
 
 
-class _InvCDF:
-    """Stand-in for torch.distributions.Categorical inside the oracle: first index whose running probability exceeds u."""
-    table_for_pass = None
-    pass_index = -1
-    step = 0
-
-    def __init__(self, logits):
-        self.logits = logits
-
-    def sample(self):
-        c = torch.softmax(self.logits.double(), -1).cumsum(-1)
-        u = _InvCDF.table_for_pass(_InvCDF.pass_index, c.shape[0])[_InvCDF.step]
-        _InvCDF.step += 1
-        return (c > u[:, None]).to(torch.uint8).argmax(-1)
-
-
 def _uniforms(pass_index, n_seq, rows=64):
     g = torch.Generator().manual_seed(900 + pass_index)
     return torch.rand(rows, n_seq, generator=g, dtype=torch.float64)
@@ -110,26 +96,12 @@ def _uniforms(pass_index, n_seq, rows=64):
 
 @pytest.mark.parametrize("temps,carry", [((0.0, 0.4), True), ((0.0, 0.8), True), ((0.0, 0.4, 0.6), False)])
 def test_transcribe_fallback_prompt_and_seek_match_unmodified_reference(env, temps, carry):
-    import oracle.whisper_ref.decoding as odec
-    import stable_whisper.whisper_word_level.original_whisper as ow
-    SP, om, stand = env["SP"], env["om"], env["stand"]
+    """The reference's sampler drew from the same ``_uniforms`` through the draw rule of stb_sample (first index whose running
+    probability exceeds u)."""
+    SP, stand = env["SP"], env["stand"]
     audio = torch.cat([SP.synth_audio(480000, seed=21), SP.synth_audio(330000, seed=22)])
-    orig_cat, orig_dec = odec.Categorical, ow.decode_stable
-    _InvCDF.table_for_pass, _InvCDF.pass_index = _uniforms, -1
-
-    def counting_decode(model, seg, options, **kw):
-        if options.temperature > 0:
-            _InvCDF.pass_index += 1
-            _InvCDF.step = 0
-        return orig_dec(model, seg, options, **kw)
-    odec.Categorical, ow.decode_stable = _InvCDF, counting_decode
-    try:
-        theirs = ow.transcribe_stable(om, audio, language="en", temperature=temps, best_of=2, condition_on_previous_text=carry,
-                                      word_timestamps=True, vad=False, suppress_silence=False, suppress_ts_tokens=False,
-                                      regroup=False, verbose=None, fp16=False, ignore_compatibility=True, sample_len=16)
-    finally:
-        odec.Categorical, ow.decode_stable = orig_cat, orig_dec
-    n_ref_passes = _InvCDF.pass_index + 1
+    ref = _golden(f"fallback|{temps}|{carry}")
+    n_ref_passes = ref["passes"]
     calls = []
 
     def source(ti, steps, n_seq):
@@ -138,7 +110,7 @@ def test_transcribe_fallback_prompt_and_seek_match_unmodified_reference(env, tem
     mine = stand.transcribe(audio, language="en", temperature=temps, best_of=2, condition_on_previous_text=carry, regroup=False,
                             sample_len=16, shard_seconds=None, batch_windows=1, uniforms=source, suppress_silence=False)
     assert len(calls) == n_ref_passes and n_ref_passes >= 2
-    da, db = mine.to_dict(), theirs.to_dict()
+    da, db = mine.to_dict(), ref
     assert len(da["segments"]) == len(db["segments"]) and len(da["segments"]) >= 2
     for sa, sb in zip(da["segments"], db["segments"]):
         assert sa["tokens"] == [int(t) for t in sb["tokens"]] and sa["seek"] == sb["seek"]
@@ -155,15 +127,12 @@ def test_transcribe_with_silence_masks_matches_unmodified_reference(env):
     only runs its silence detector with ``suppress_silence=True`` (``vad=vad if suppress_silence else None``, :428), which also
     re-times the words afterwards (``Segment.suppress_silence``, out of scope here): tokens, seeks and word token groups are
     applied here through the reference's own class, api.transcribe): everything is compared, word boundaries included."""
-    import stable_whisper.whisper_word_level.original_whisper as ow
-    SP, om, stand = env["SP"], env["om"], env["stand"]
+    SP, stand = env["SP"], env["stand"]
     audio = torch.cat([SP.synth_gapped_audio(480000, seed=61), torch.zeros(200000), SP.synth_gapped_audio(300000, seed=62)])
-    theirs = ow.transcribe_stable(om, audio, language="en", temperature=0.0, condition_on_previous_text=True, word_timestamps=True,
-                                  vad=False, suppress_silence=True, suppress_ts_tokens=True, regroup=False, verbose=None,
-                                  fp16=False, ignore_compatibility=True, sample_len=16)
+    theirs = _golden("silence_masks")
     mine = stand.transcribe(audio, language="en", temperature=0.0, condition_on_previous_text=True, regroup=False,
                             sample_len=16, shard_seconds=None, batch_windows=1, suppress_ts_tokens=True)
-    da, db = mine.to_dict(), theirs.to_dict()
+    da, db = mine.to_dict(), theirs
     assert len(da["segments"]) == len(db["segments"]) and len(da["segments"]) >= 1
     n_moved = 0
     for sa, sb in zip(da["segments"], db["segments"]):
@@ -184,16 +153,13 @@ def test_transcribe_nonspeech_skip_and_avg_prob_threshold_match_unmodified_refer
     """The two remaining seek controls of the transcribe loop: ``nonspeech_skip`` (a long silence ends the window where it
     starts, or is skipped when it leads the window; original_whisper.py:512-526) and ``avg_prob_threshold`` (:665-675,693-694).
     Audio: a long leading silence, speech, a long inner silence, speech.  Everything vs the reference, re-timed words included."""
-    import stable_whisper.whisper_word_level.original_whisper as ow
-    SP, om, stand = env["SP"], env["om"], env["stand"]
+    SP, stand = env["SP"], env["stand"]
     audio = torch.cat([torch.zeros(90000), SP.synth_audio(150000, seed=71), torch.zeros(100000), SP.synth_audio(260000, seed=72),
                        torch.zeros(70000), SP.synth_audio(120000, seed=73)])
-    theirs = ow.transcribe_stable(om, audio, language="en", temperature=0.0, condition_on_previous_text=False, word_timestamps=True,
-                                  vad=False, suppress_silence=True, suppress_ts_tokens=False, regroup=False, verbose=None,
-                                  fp16=False, ignore_compatibility=True, sample_len=16, **opts)
+    theirs = _golden("seek_controls|" + json.dumps(opts, sort_keys=True))
     mine = stand.transcribe(audio, language="en", temperature=0.0, condition_on_previous_text=False, regroup=False,
                             sample_len=16, shard_seconds=None, batch_windows=1, **opts)
-    da, db = mine.to_dict(), theirs.to_dict()
+    da, db = mine.to_dict(), theirs
     assert [s["seek"] for s in da["segments"]] == [s["seek"] for s in db["segments"]]
     assert len(da["segments"]) == len(db["segments"])
     for sa, sb in zip(da["segments"], db["segments"]):
@@ -209,18 +175,15 @@ def test_clip_timestamps_match_unmodified_reference(env, parallel):
     """``clip_timestamps`` (the reference's load_sections): only the given sections are transcribed, a window never crosses a
     section end.  Walked as ONE sequential shard (prompt carried across clips, exactly the reference) and as independent
     shards batched side by side (SURVEY.md section 8e: equal to the reference with condition_on_previous_text=False)."""
-    import stable_whisper.whisper_word_level.original_whisper as ow
-    SP, om, stand = env["SP"], env["om"], env["stand"]
+    SP, stand = env["SP"], env["stand"]
     audio = torch.cat([SP.synth_audio(480000, seed=81), SP.synth_audio(480000, seed=82), SP.synth_audio(200000, seed=83)])
     clips = [2.5, 21.0, 30.0, 65.5, 66.0]                      # two closed clips (one longer than a window) and an open one
     carry = not parallel
-    theirs = ow.transcribe_stable(om, audio, language="en", temperature=0.0, condition_on_previous_text=carry, word_timestamps=True,
-                                  vad=False, suppress_silence=False, suppress_ts_tokens=False, regroup=False, verbose=None,
-                                  fp16=False, ignore_compatibility=True, sample_len=16, clip_timestamps=clips)
+    theirs = _golden(f"clip|{parallel}")
     mine = stand.transcribe(audio, language="en", temperature=0.0, condition_on_previous_text=carry, regroup=False,
                             sample_len=16, shard_seconds=30.0 if parallel else None, batch_windows=4, clip_timestamps=clips,
                             suppress_silence=False)
-    da, db = mine.to_dict(), theirs.to_dict()
+    da, db = mine.to_dict(), theirs
     assert [s["seek"] for s in da["segments"]] == [s["seek"] for s in db["segments"]] and len(da["segments"]) >= 3
     for sa, sb in zip(da["segments"], db["segments"]):
         assert sa["tokens"] == [int(t) for t in sb["tokens"]]
@@ -235,28 +198,23 @@ def test_transcribe_word_timestamp_variants_match_unmodified_reference(env, vari
     635-651): the "new" aligner, dynamic heads, ``extra_models``, ``char_split`` (popped from the shared dict by the first
     window, as in the reference) and custom punctuation sets."""
     import oracle.whisper_ref as W
-    import stable_whisper.whisper_word_level.original_whisper as ow
     from standin import OracleBackedModel
-    SP, om, stand = env["SP"], env["om"], env["stand"]
+    SP, stand = env["SP"], env["stand"]
     audio = torch.cat([SP.synth_audio(480000, seed=91), SP.synth_audio(250000, seed=92)])
-    ref_kw, kw = {}, {}
     if variant == "new":
-        ref_kw, kw = dict(aligner="new"), dict(aligner="new")
+        kw = dict(aligner="new")
     elif variant == "dynamic":
-        ref_kw, kw = dict(dynamic_heads="3,2"), dict(dynamic_heads="3,2")
+        kw = dict(dynamic_heads="3,2")
     elif variant == "extra_models":
-        om2 = W.build_model("tiny.en", seed=4)
-        ref_kw, kw = dict(extra_models=[om2]), dict(extra_models=[OracleBackedModel(om2)])
+        kw = dict(extra_models=[OracleBackedModel(W.build_model("tiny.en", seed=4))])
     elif variant == "char_split":
-        ref_kw, kw = dict(aligner={"char_split": True}), dict(aligner={"char_split": True})
+        kw = dict(aligner={"char_split": True})
     else:
-        ref_kw = kw = dict(prepend_punctuations="(", append_punctuations=".,")
-    theirs = ow.transcribe_stable(om, audio, language="en", temperature=0.0, condition_on_previous_text=False, word_timestamps=True,
-                                  vad=False, suppress_silence=False, suppress_ts_tokens=False, regroup=False, verbose=None,
-                                  fp16=False, ignore_compatibility=True, sample_len=16, **ref_kw)
+        kw = dict(prepend_punctuations="(", append_punctuations=".,")
+    theirs = _golden(f"word_variant|{variant}")
     mine = stand.transcribe(audio, language="en", temperature=0.0, condition_on_previous_text=False, regroup=False,
                             sample_len=16, shard_seconds=None, batch_windows=1, suppress_silence=False, **kw)
-    da, db = mine.to_dict(), theirs.to_dict()
+    da, db = mine.to_dict(), theirs
     assert [s["seek"] for s in da["segments"]] == [s["seek"] for s in db["segments"]] and len(da["segments"]) >= 2
     for sa, sb in zip(da["segments"], db["segments"]):
         assert sa["tokens"] == [int(t) for t in sb["tokens"]] and sa["start"] == sb["start"] and sa["end"] == sb["end"]

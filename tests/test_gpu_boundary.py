@@ -2,10 +2,11 @@
 
 B2: the whisper model-object protocol of shim.py -- forward hooks on ``decoder.blocks[i].cross_attn`` see the layer's ``qk``,
     ``model(mel, tokens)`` broadcasts one token row, the ``kv_cache`` protocol decodes incrementally, ``detect_language``.
-B0/B1 (when ``baseline/_ref`` holds the installed reference package; it travels to the GPU box with the snapshot): the
-    UNMODIFIED ``Aligner`` / ``Refiner`` drive the B200 closures through ``model.align`` / ``align_words`` / ``refine`` /
-    ``locate``; the results must equal what the reference's own entry points produce over the CPU oracle model
-    (words +-20 ms, probabilities 2e-3)."""
+B0/B1 (when ``build()`` installed the reference package into ``oracle/_ref/``, oracle/reference_install.py): the UNMODIFIED
+    ``Aligner`` / ``Refiner`` drive the B200 closures through ``model.align`` / ``align_words`` / ``refine``; the results must equal what the reference's own entry
+    points produce over the CPU oracle model (words +-20 ms, probabilities 2e-3).
+``locate``, ``transcribe`` and the word-timestamp variants are compared with what the unmodified reference produced over the
+    CPU oracle model on the same seeded inputs (tests/golden/reference_results.json, oracle/make_golden_reference.py)."""
 import copy
 import os
 import sys
@@ -16,7 +17,16 @@ import torch
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_INSTALL = os.path.join(ROOT, "baseline", "_ref")
+GOLD = os.path.join(ROOT, "tests", "golden", "reference_results.json")
+
+
+def _golden(*keys):
+    import json
+    with open(GOLD) as f:
+        d = json.load(f)
+    for k in keys:
+        d = d[k]
+    return d
 
 
 def _gpu():
@@ -80,16 +90,28 @@ def test_protocol_hooks_logits_and_kv_cache():
     assert abs(probs[top] - probs_ref[top]) <= 2e-3 * probs_ref[top]
 
 
-@pytest.fixture(scope="module")
+@pytest.fixture
 def ref_env():
+    """The reference package importable (from oracle/_ref/) for the test that drives its control plane, and no longer
+    afterwards: the other tests check this package's own result classes."""
     _gpu()
-    if not os.path.isdir(os.path.join(REF_INSTALL, "stable_whisper")):
-        pytest.skip("baseline/_ref (pip --target install of the reference) is not present")
+    from oracle import reference_install
+    root = reference_install.path()
+    if root is None:
+        pytest.skip("the reference package (stable-ts) is not installed in oracle/_ref/")
     import oracle.whisper_ref as W
     W.install_as_whisper()                    # the reference imports `whisper`; the CPU oracle restates it
-    if REF_INSTALL not in sys.path:
-        sys.path.insert(0, REF_INSTALL)
-    import stable_whisper  # noqa: F401
+    sys.path.insert(0, root)
+    try:
+        import stable_whisper  # noqa: F401
+        yield _ref_inputs()
+    finally:
+        sys.path.remove(root)
+        for name in [m for m in sys.modules if m == "stable_whisper" or m.startswith("stable_whisper.")]:
+            del sys.modules[name]
+
+
+def _ref_inputs():
     from oracle import stable_path as SP
     W, om, gm = _models()
     otk = W.tokenizer.get_tokenizer(True, num_languages=om.num_languages, language="en", task="transcribe")
@@ -135,12 +157,14 @@ def test_unmodified_aligner_and_refiner_over_b200_kernels(ref_env):
 
 
 @pytest.mark.parametrize("mode,thr", [(2, 0.5), (0, 0.0), (1, 0.0)])
-def test_locate_matches_reference_over_oracle(ref_env, mode, thr):
-    import stable_whisper.alignment as ref_align
-    om, gm, audio = ref_env["om"], ref_env["gm"], ref_env["audio"]
+def test_locate_matches_reference_over_oracle(mode, thr):
+    _gpu()
+    from oracle import stable_path as SP
+    _, _, gm = _models()
+    audio = torch.cat([SP.synth_gapped_audio(400000, seed=11), SP.synth_audio(300000, seed=12)])
     text = [700, 901, 333]
     kw = dict(count=3, mode=mode, probability_threshold=thr, exact_token=True, max_token_per_seg=8)
-    theirs = ref_align.locate(om, audio, text, "en", verbose=None, **kw)
+    theirs = _golden("boundary", "locate", f"{mode}|{thr}")
     mine = gm.locate(audio, text, "en", **kw)
     assert len(mine) == len(theirs) and len(mine) > 0
     for a, b in zip(mine, theirs):
@@ -150,7 +174,7 @@ def test_locate_matches_reference_over_oracle(ref_env, mode, thr):
             assert abs(a["end"] - b["end"]) <= 0.0201
             assert [w["tokens"] for w in a["duration_window_word"]] == [w["tokens"] for w in b["duration_window_word"]]
         else:
-            da, db = a.to_dict(), b.to_dict()
+            da, db = a.to_dict(), b
             assert [w["tokens"] for w in da["words"]] == [w["tokens"] for w in db["words"]]
             assert max(max(abs(x["start"] - y["start"]), abs(x["end"] - y["end"])) for x, y in zip(da["words"], db["words"])) <= 0.0201
 
@@ -172,59 +196,27 @@ def test_transcribe_method_returns_result_object():
         assert [s["tokens"] for s in mine[: len(ref)]] == [[t for t in s["tokens"] if t < otk.eot] for s in ref]
 
 
-class _InvCDF:
-    """Test-only stand-in for ``torch.distributions.Categorical`` inside the CPU oracle: the draw rule of ``stb_sample`` (first
-    index whose running probability exceeds u) fed from the same table of uniforms as the GPU path."""
-    table_for_pass = None        # callable(pass_index, n_seq) -> fp64 [rows, n_seq]
-    pass_index = -1
-    step = 0
-
-    def __init__(self, logits):
-        self.logits = logits
-
-    def sample(self):
-        c = torch.softmax(self.logits.double(), -1).cumsum(-1)
-        u = _InvCDF.table_for_pass(_InvCDF.pass_index, c.shape[0])[_InvCDF.step]
-        _InvCDF.step += 1
-        return (c > u[:, None]).to(torch.uint8).argmax(-1)
-
-
 def _extreme_uniforms(pass_index, n_seq, rows=64):
     """u = 0 (first token with probability > 0) or 1 - 2^-24 (last one), alternating over sequences and passes: the drawn
     token then depends on the logit FILTERS only, never on a near-tie of two running sums, so the CPU oracle and the GPU
-    draw the same tokens although their logits differ by ~1e-5 relative."""
+    draw the same tokens although their logits differ by ~1e-5 relative.  oracle/make_golden_reference.py fed the same
+    table, through the draw rule of ``stb_sample`` (first index whose running probability exceeds u), to the reference."""
     hi = 1.0 - 2.0 ** -24
     row = torch.tensor([0.0 if (s + pass_index) % 2 == 0 else hi for s in range(n_seq)], dtype=torch.float64)
     return row.repeat(rows, 1)
 
 
 @pytest.mark.parametrize("temps,carry", [((0.0, 0.4), True), ((0.0, 0.8), True), ((0.0, 0.4), False)])
-def test_transcribe_fallback_and_prompt_carry_match_unmodified_reference(ref_env, temps, carry):
-    """Whole-audio ``transcribe`` (one sequential shard) == the UNMODIFIED transcribe_stable over the CPU oracle model:
-    temperature fallback with best_of draws (original_whisper.py:349-393), prompt carry-over and its reset after a window decoded
-    above temperature 0.5 (:533,696-698), data-dependent seek (:703-710)."""
-    import oracle.whisper_ref.decoding as odec
-    import stable_whisper.whisper_word_level.original_whisper as ow
+def test_transcribe_fallback_and_prompt_carry_match_unmodified_reference(temps, carry):
+    """Whole-audio ``transcribe`` (one sequential shard) == the UNMODIFIED transcribe_stable over the CPU oracle model, its
+    sampler drawing from the same ``_extreme_uniforms``: temperature fallback with best_of draws (original_whisper.py:349-393),
+    prompt carry-over and its reset after a window decoded above temperature 0.5 (:533,696-698), data-dependent seek (:703-710)."""
+    _gpu()
     from oracle import stable_path as SP
-    W, om, gm = _models("tiny.en", seed=3)
+    _, _, gm = _models("tiny.en", seed=3)
     audio = torch.cat([SP.synth_audio(480000, seed=21), SP.synth_audio(330000, seed=22)])
-    # --- reference side
-    orig_cat, orig_dec = odec.Categorical, ow.decode_stable
-    _InvCDF.table_for_pass, _InvCDF.pass_index = _extreme_uniforms, -1
-
-    def counting_decode(model, seg, options, **kw):
-        if options.temperature > 0:
-            _InvCDF.pass_index += 1
-            _InvCDF.step = 0
-        return orig_dec(model, seg, options, **kw)
-    odec.Categorical, ow.decode_stable = _InvCDF, counting_decode
-    try:
-        theirs = ow.transcribe_stable(om, audio, language="en", temperature=temps, best_of=2, condition_on_previous_text=carry,
-                                      word_timestamps=True, vad=False, suppress_silence=False, suppress_ts_tokens=False,
-                                      regroup=False, verbose=None, fp16=False, ignore_compatibility=True, sample_len=24)
-    finally:
-        odec.Categorical, ow.decode_stable = orig_cat, orig_dec
-    n_ref_passes = _InvCDF.pass_index + 1
+    ref = _golden("transcribe", f"fallback_extreme|{temps}|{carry}")
+    n_ref_passes = ref["passes"]
     # --- B200 side: same uniforms, pass by pass
     calls = []
 
@@ -234,9 +226,9 @@ def test_transcribe_fallback_and_prompt_carry_match_unmodified_reference(ref_env
     mine = gm.transcribe(audio, language="en", temperature=temps, best_of=2, condition_on_previous_text=carry, regroup=False,
                          sample_len=24, shard_seconds=None, batch_windows=1, uniforms=source, suppress_silence=False)
     assert len(calls) == n_ref_passes and n_ref_passes >= 1
-    da, db = mine.to_dict(), theirs.to_dict()
-    assert len(da["segments"]) == len(db["segments"])
-    for sa, sb in zip(da["segments"], db["segments"]):
+    da = mine.to_dict()
+    assert len(da["segments"]) == len(ref["segments"])
+    for sa, sb in zip(da["segments"], ref["segments"]):
         assert sa["tokens"] == [int(t) for t in sb["tokens"]] and sa["seek"] == sb["seek"]
         assert sa["temperature"] == sb["temperature"]
         assert abs(sa["avg_logprob"] - sb["avg_logprob"]) < 1e-3
@@ -248,11 +240,11 @@ def test_transcribe_fallback_and_prompt_carry_match_unmodified_reference(ref_env
 
 
 @pytest.mark.parametrize("variant", ["char_split", "extra_models", "extra_models_dynamic"])
-def test_timing_variants_match_unmodified_reference(ref_env, variant):
+def test_timing_variants_match_unmodified_reference(variant):
     """``extra_models`` and the "new" aligner's ``char_split`` (timing.py:177-189,240-253,380-390,442-444) through
     ``add_word_timestamps_stable`` on the kernels vs the unmodified function over the CPU oracle models."""
+    _gpu()
     import oracle.whisper_ref as W
-    import stable_whisper.timing as ref_timing
     from oracle import stable_path as SP
     from stable_ts_b200.model import from_oracle
     from stable_ts_b200.timing import add_word_timestamps_stable
@@ -262,17 +254,14 @@ def test_timing_variants_match_unmodified_reference(ref_env, variant):
     otk = W.tokenizer.get_tokenizer(True, num_languages=om.num_languages, language="en", task="transcribe")
     tk = get_tokenizer(gm, language="en", task="transcribe", synthetic=True)
     audio = SP.synth_audio(400000, seed=51)
-    mel = W.pad_or_trim(W.log_mel_spectrogram(audio, om.dims.n_mels, padding=80000), 3000)
     script = SP.synth_token_script(36, otk.eot, seed=52)
-    theirs = [dict(seek=0.0, tokens=script[:20]), dict(seek=0.0, tokens=script[20:])]
-    mine = copy.deepcopy(theirs)
-    kw_ref, kw = {}, {}
+    mine = [dict(seek=0.0, tokens=script[:20]), dict(seek=0.0, tokens=script[20:])]
     if variant == "char_split":
-        kw_ref, kw = dict(aligner={"char_split": True}), dict(aligner={"char_split": True})
+        kw, key = dict(aligner={"char_split": True}), "char_split"
     else:
         dyn = "4,2" if variant.endswith("dynamic") else None
-        kw_ref, kw = dict(extra_models=[om2], dynamic_heads=dyn), dict(extra_models=[gm2], dynamic_heads=dyn)
-    ref_timing.add_word_timestamps_stable(segments=theirs, model=om, tokenizer=otk, mel=mel, num_samples=400000, **kw_ref)
+        kw, key = dict(extra_models=[gm2], dynamic_heads=dyn), f"extra_models_{dyn}"
+    theirs = _golden("timing_variants", key)
     add_word_timestamps_stable(segments=mine, model=gm, tokenizer=tk, audio=audio, num_samples=400000, **kw)
     n, worst = 0, 0.0
     for a, b in zip(mine, theirs):

@@ -67,11 +67,10 @@ def test_product_host_half_matches_oracle():
 
 
 def test_reference_demo_wav_header_if_present():
-    """examples/demo.wav of the reference (44.1 kHz stereo s16; BASELINE config 1) parses; build container only."""
+    """examples/demo.wav of the reference (44.1 kHz stereo s16; BASELINE config 1) parses: its first 0.1 s, header chunks
+    kept as they are (tests/golden/demo_head.wav, oracle/make_golden_reference.py)."""
     import os
-    p = "/root/reference/examples/demo.wav"
-    if not os.path.exists(p):
-        pytest.skip("reference tree absent")
+    p = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "demo_head.wav")
     from stable_ts_b200 import audio_io as A
     rate, ch, fmt, payload = A.parse_wav(open(p, "rb").read())
     assert (rate, ch, fmt) == (44100, 2, 0)

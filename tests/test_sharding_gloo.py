@@ -107,16 +107,11 @@ def test_gathered_words_lazy_view_equals_eager_unpack():
             assert [d["tokens"] for d in eager[per * r + w]] == [d["tokens"] for d in res[w]]
 
 
-def test_gathered_records_rebuild_the_result_wire_format():
-    """SURVEY.md section 8f row 4: the gather payload -> dict with WhisperResult.to_dict's keys; loads in the stand-in result
-    class and, in the build container, in the reference's own WhisperResult."""
-    import os
-    import sys
+def gathered_result_dict(world=2, per=3):
+    """The result dict rebuilt from the gathered word records of `world` ranks with `per` windows each (-> (dict, n_words))."""
     from stable_ts_b200 import sharding as S
-    from stable_ts_b200.result import WhisperResult
     from stable_ts_b200.tokenizer import Tokenizer
     tk = Tokenizer(True, 99, "en", "transcribe")
-    world, per = 2, 3
     res = []
     for w in range(per):
         ws = _fake_words(100 + w)
@@ -127,17 +122,26 @@ def test_gathered_records_rebuild_the_result_wire_format():
     bufs = [S.pack_records([[dict(w, start=w["start"] + 30.0 * (per * r + i), end=w["end"] + 30.0 * (per * r + i)) for w in ws]
                             for i, ws in enumerate(res)], per * r, cap_w, cap_t) for r in range(world)]
     g = S.unpack_records(bufs, per * world, cap_w, lazy=True, tokenizer=tk)
-    d = S.gathered_to_result(g, tk)
-    n_words = world * sum(len(w) for w in res)
+    return S.gathered_to_result(g, tk), world * sum(len(w) for w in res)
+
+
+def test_gathered_records_rebuild_the_result_wire_format():
+    """SURVEY.md section 8f row 4: the gather payload -> dict with WhisperResult.to_dict's keys; loads in the stand-in result
+    class exactly as in the reference's own WhisperResult (tests/golden/reference_results.json, written by the unmodified
+    reference from the same dict)."""
+    import json
+    from stable_ts_b200.result import WhisperResult
+    from stable_ts_b200.tokenizer import Tokenizer
+    tk = Tokenizer(True, 99, "en", "transcribe")
+    d, n_words = gathered_result_dict()
     assert d["language"] == "en" and sum(len(s["words"]) for s in d["segments"]) == n_words
     for s in d["segments"]:
         assert s["text"] == "".join(w["word"] for w in s["words"]) == tk.decode(s["tokens"])
         assert s["start"] == s["words"][0]["start"] and s["end"] == s["words"][-1]["end"] and s["seek"] == 30.0 * (s["start"] // 30.0)
     mine = WhisperResult(d)
     assert len(mine.all_words()) == n_words and mine.text == d["text"]
-    if os.path.isdir("/root/reference"):
-        sys.path.insert(0, "/root/reference")
-        import stable_whisper
-        theirs = stable_whisper.WhisperResult(d)
-        assert theirs.text == mine.text and len(theirs.all_words()) == n_words
-        assert [w.to_dict() for w in theirs.all_words()] == [w.to_dict() for w in mine.all_words()]
+    gold = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_results.json")
+    with open(gold) as f:
+        theirs = json.load(f)["sharding_result"]
+    assert theirs["text"] == mine.text and len(theirs["words"]) == n_words
+    assert theirs["words"] == [w.to_dict() for w in mine.all_words()]

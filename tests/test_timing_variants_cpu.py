@@ -1,24 +1,19 @@
 """``extra_models`` and the "new" aligner's ``char_split`` (stable_whisper/timing.py:177-189, 240-253, 380-390, 442-444): the host
-logic of stable_ts_b200.timing over the oracle-backed stand-in vs the UNMODIFIED ``add_word_timestamps_stable`` over the same
-oracle models.  (Build container only; the kernels behind the stand-in's methods are pinned by the -m gpu tests.)"""
+logic of stable_ts_b200.timing over the oracle-backed stand-in vs what the UNMODIFIED ``add_word_timestamps_stable`` returned
+over the same oracle models (tests/golden/reference_results.json, oracle/make_golden_reference.py).  The kernels behind the
+stand-in's methods are pinned by the -m gpu tests."""
 import copy
+import json
 import os
-import sys
 
 import pytest
-import torch
 
-REFERENCE = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference tree only exists in the build container")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_results.json")
 
 
 @pytest.fixture(scope="module")
 def env():
     import oracle.whisper_ref as W
-    W.install_as_whisper()
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-    import stable_whisper.timing as ref_timing
     from oracle import stable_path as SP
     from standin import OracleBackedModel
     from stable_ts_b200.tokenizer import get_tokenizer
@@ -27,21 +22,18 @@ def env():
     otk = W.tokenizer.get_tokenizer(True, num_languages=om.num_languages, language="en", task="transcribe")
     tk = get_tokenizer(stand, language="en", task="transcribe", synthetic=True)
     audio = SP.synth_audio(400000, seed=51)
-    mel = W.pad_or_trim(W.log_mel_spectrogram(audio, om.dims.n_mels, padding=80000), 3000)
     script = SP.synth_token_script(36, otk.eot, seed=52)
     segs = [dict(seek=0.0, tokens=script[:20]), dict(seek=0.0, tokens=script[20:])]
-    return dict(W=W, ref=ref_timing, om=om, om2=om2, stand=stand, stand2=stand2, otk=otk, tk=tk, audio=audio, mel=mel, segs=segs)
+    with open(GOLD) as f:
+        gold = json.load(f)["timing_variants"]
+    return dict(stand=stand, stand2=stand2, tk=tk, audio=audio, segs=segs, gold=gold)
 
 
-def _run_both(env, **kw):
+def _run_both(env, key, **kw):
     from stable_ts_b200.timing import add_word_timestamps_stable
-    theirs, mine = copy.deepcopy(env["segs"]), copy.deepcopy(env["segs"])
-    ref_kw = {k: copy.deepcopy(v) if isinstance(v, dict) else v for k, v in kw.items()}
-    if "extra_models" in ref_kw:
-        ref_kw["extra_models"] = [env["om2"]]
+    theirs, mine = env["gold"][key], copy.deepcopy(env["segs"])
+    if "extra_models" in kw:
         kw["extra_models"] = [env["stand2"]]
-    env["ref"].add_word_timestamps_stable(segments=theirs, model=env["om"], tokenizer=env["otk"], mel=env["mel"],
-                                          num_samples=400000, **ref_kw)
     add_word_timestamps_stable(segments=mine, model=env["stand"], tokenizer=env["tk"], audio=env["audio"], num_samples=400000, **kw)
     n = 0
     for a, b in zip(mine, theirs):
@@ -56,10 +48,10 @@ def _run_both(env, **kw):
 
 
 def test_char_split_matches_reference(env):
-    assert _run_both(env, aligner={"char_split": True}) > 5
-    assert _run_both(env, aligner={"char_split": True, "topk": 10}) > 5
+    assert _run_both(env, "char_split", aligner={"char_split": True}) > 5
+    assert _run_both(env, "char_split_topk10", aligner={"char_split": True, "topk": 10}) > 5
 
 
 @pytest.mark.parametrize("dyn", [None, 4, "4,2"])
 def test_extra_models_match_reference(env, dyn):
-    assert _run_both(env, extra_models=True, dynamic_heads=dyn) > 5
+    assert _run_both(env, f"extra_models_{dyn}", extra_models=True, dynamic_heads=dyn) > 5
